@@ -8,6 +8,7 @@ offline), inputs synthetic.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference ...                           # the reference's algorithm on the host CPU (oracle port)
+    python bench.py ... --dump-outputs DIR                         # also write the last timed step's outputs as DIR/*.npy
 
 N > 1 (torchrun): sampling does not exchange anything between images, so ranks are independent replicas
 ("replicas only", DESIGN.md §Multi-GPU); value = N * K steps / max-over-ranks time.
@@ -115,6 +116,31 @@ def measured_peaks():
         d = json.load(open(path))
         return d.get("bf16_tflops_sustained", 1412.1), d.get("hbm_gbs", 6569.6), "measured (MEASURED_PEAKS.json)"
     return 1400.0, 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_MAX_ELEMENTS = 1 << 20  # a larger output is dumped as a sample of this many elements
+DUMP_MAX_BYTES = 64 << 20
+
+
+def host_copy(t):
+    """fp32 host copy of an output for --dump-outputs: the whole tensor, or the same seeded sample of its elements in
+    every run when it is larger than DUMP_MAX_ELEMENTS."""
+    t = t.detach()
+    if t.numel() > DUMP_MAX_ELEMENTS:
+        idx = torch.randint(t.numel(), (DUMP_MAX_ELEMENTS,), generator=torch.Generator().manual_seed(0))
+        t = t.reshape(-1)[idx.to(t.device)]
+    return t.float().cpu()
+
+
+def write_outputs(path, outputs):
+    """outputs {name: host tensor} -> path/<name>.npy (float32), so that two builds can be compared output for output"""
+    import numpy as np
+    arrays = {name: t.numpy().astype(np.float32) for name, t in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"outputs to dump take {total} bytes, more than {DUMP_MAX_BYTES}"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 def cpu_reference_pass(model_state, threads, n_images=1, seed=1):
@@ -295,9 +321,10 @@ TRAIN_BATCH = 16
 TF_PER_IMAGE_TRAIN = 2.11  # algorithmically necessary TFLOP per image of one finetune step at rank 128 (BASELINE.md §2)
 
 
-def run_train(args, rank, local_rank, world, device):
+def run_train(args, rank, local_rank, world, device, outputs=None):
     """BASELINE.json configs[2]: ctrlora_finetune_sd15_rank128 training step, synthetic pairs, batch 16 per GPU,
-    data-parallel with ONE NCCL all-reduce of the flat trainable-gradient buffer per step.  Returns a dict."""
+    data-parallel with ONE NCCL all-reduce of the flat trainable-gradient buffer per step.  Returns a dict; the last timed
+    step's loss and the trained parameters go to `outputs` when it is given."""
     import torch.distributed as dist
     from ctrlora_b200 import dropin
     dropin.activate()
@@ -334,6 +361,8 @@ def run_train(args, rank, local_rank, world, device):
         loss = trainer.step(*dev)
     e1.record()
     barrier()
+    if outputs is not None:  # before the next step overwrites the graph's loss buffer and the parameters
+        outputs.update(train_loss=host_copy(loss), train_params=host_copy(trainer.G.flat_p))
     ms_dev = e0.elapsed_time(e1)
     loss_host = torch.empty(1).pin_memory()
     h2d = sum(host[k].numel() * host[k].element_size() for k in order)
@@ -373,10 +402,11 @@ TF_PER_IMAGE_PRETRAIN = 2.33  # the finetune step's 2.11 TF + dense weight gradi
 # (= their forward cost: conv 122.4 + Linear 95.8 GF, SURVEY.md §8d) -- algorithmically necessary work per image
 
 
-def run_pretrain(args, rank, local_rank, world, device):
+def run_pretrain(args, rank, local_rank, world, device, outputs=None):
     """BASELINE.json configs[3]: ctrlora_pretrain_sd15_9tasks_rank128, one task per mini-batch from the multi-task
     schedule (per-rank un-seeded permutations in the reference -> ranks generally train different tasks in a step), batch 8
-    per GPU (global 64 on 8 GPUs).  All ControlNet parameters + the task's LoRA set are trained."""
+    per GPU (global 64 on 8 GPUs).  All ControlNet parameters + the task's LoRA set are trained.  The last timed step's
+    loss and the trained parameters go to `outputs` when it is given."""
     import numpy as np
     import torch.distributed as dist
     from ctrlora_b200 import dropin
@@ -417,6 +447,8 @@ def run_pretrain(args, rank, local_rank, world, device):
         loss = trainer.step(*dev, task=next(it))
     e1.record()
     barrier()
+    if outputs is not None:
+        outputs.update(pretrain_loss=host_copy(loss), pretrain_params=host_copy(trainer.G.flat_p))
     ms_dev = e0.elapsed_time(e1)
     loss_host = torch.empty(1).pin_memory()
     h2d = sum(host[k].numel() * host[k].element_size() for k in order)
@@ -501,8 +533,16 @@ def main():
     ap.add_argument("--workload", default="sample+train", choices=["sample", "train", "sample+train", "pretrain"],
                     help="sample: configs[1] DDIM step (the headline line); train: configs[2] finetune step; default: both, "
                          "the training result rides in the line's 'train' key")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (DDIM x_prev / pred_x0; training loss and a fixed sample "
+                         "of the trained parameters) to DIR/<name>.npy; the inputs are seeded, so two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank, local_rank, world = dist_env()
+    outputs = {} if args.dump_outputs and rank == 0 else None
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args, rank, world)
@@ -519,7 +559,9 @@ def main():
     from ctrlora_b200 import dropin, ops
     dropin.activate()
     if args.workload == "pretrain":
-        res = run_pretrain(args, rank, local_rank, world, device)
+        res = run_pretrain(args, rank, local_rank, world, device, outputs)
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         if rank == 0:
             line = {"metric": res["metric"], "value": res["value"], "unit": res["unit"], "n_gpus": world, "steps": args.steps,
                     "warmup": args.warmup, "ms_per_step": res["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -533,7 +575,9 @@ def main():
             dist.destroy_process_group()
         return
     if args.workload == "train":
-        res = run_train(args, rank, local_rank, world, device)
+        res = run_train(args, rank, local_rank, world, device, outputs)
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         if rank == 0:
             line = {"metric": res["metric"], "value": res["value"], "unit": res["unit"], "n_gpus": world, "steps": args.steps,
                     "warmup": args.warmup, "ms_per_step": res["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -601,11 +645,13 @@ def main():
     x = dev["x"]
     with sampler.run_mode():  # the K steps of a sampling run share their conditioning (as in DDIMSampler.sample)
         for i in range(args.steps):
-            x, _ = step(i, x)
+            x, pred_x0 = step(i, x)
     e1.record()
     barrier()
     ms_dev = e0.elapsed_time(e1)
     clk = clocks.stop()
+    if outputs is not None:
+        outputs.update(x_prev=host_copy(x), pred_x0=host_copy(pred_x0))
 
     # ---- (2) end to end through the public API with host buffers: H2D of the step's inputs, D2H of its result
     out_host = torch.empty(BATCH, 4, LATENT, LATENT).pin_memory()
@@ -647,7 +693,9 @@ def main():
     if "train" in args.workload:
         del sampler, model
         torch.cuda.empty_cache()
-        train_result = run_train(args, rank, local_rank, world, device)
+        train_result = run_train(args, rank, local_rank, world, device, outputs)
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     if rank == 0:
         peak_tf, peak_hbm, peak_src = measured_peaks()
         value = world * args.steps / (ms_dev / 1e3)

@@ -14,12 +14,13 @@ DESIGN.md §4):
 i.e. rounding the tensor-core OPERANDS to fp16 alone costs 1.4e-3 on this random-init network; the accumulated
 residual-stream rounding adds 11 %.  An fp32 residual stream would not bring the end-to-end figure under 1e-3.
 """
-import sys, time
+import os, sys, time
 import torch, torch.nn.functional as F
-sys.path.insert(0, '/root/repo')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 from oracle import ctrlora_oracle as O, synth
 torch.set_num_threads(32)
-g = torch.load('/root/repo/tests/golden/sd15_rank128_golden.pt', weights_only=False)
+g = torch.load(os.path.join(ROOT, 'tests', 'golden', 'sd15_rank128_golden.pt'), weights_only=False)
 seed = g['seed']
 s = synth.synth_state_dict(g['control_shapes'], seed, 'control_model.')
 u = synth.synth_state_dict(g['unet_shapes'], seed, 'model.diffusion_model.')

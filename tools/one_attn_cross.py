@@ -1,9 +1,10 @@
 """One cross-attention shape (77 context tokens, 64x64 level), a few launches (for ncu --set full)."""
+import os
 import sys
 
 import torch
 
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ctrlora_b200 import ops  # noqa: E402
 from tools.profile_kernels import rnd  # noqa: E402
 

@@ -1,9 +1,10 @@
 """One GroupNorm shape, a few launches (for ncu --set full): python tools/one_gn.py H C"""
+import os
 import sys
 
 import torch
 
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ctrlora_b200 import ops  # noqa: E402
 from tools.profile_kernels import rnd  # noqa: E402
 

@@ -8,12 +8,13 @@ model.diffusion_model.{input_blocks.i, middle_block, output_blocks.i, out}), eve
 rounding errors add in variance, so err_g^2 is block g's share of the end-to-end error^2; the table says where a
 two-term (hi + lo) fp16 split of the tensor-core operands buys the most per GEMM flop.
 """
-import json, sys, time
+import json, os, sys, time
 import torch, torch.nn.functional as F
-sys.path.insert(0, '/root/repo')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 from oracle import ctrlora_oracle as O, synth
 torch.set_num_threads(8)
-g = torch.load('/root/repo/tests/golden/sd15_rank128_golden.pt', weights_only=False)
+g = torch.load(os.path.join(ROOT, 'tests', 'golden', 'sd15_rank128_golden.pt'), weights_only=False)
 seed = g['seed']
 s = synth.synth_state_dict(g['control_shapes'], seed, 'control_model.')
 u = synth.synth_state_dict(g['unet_shapes'], seed, 'model.diffusion_model.')
@@ -151,7 +152,7 @@ def run():
 
 
 if __name__ == '__main__':
-    out_path = sys.argv[1] if len(sys.argv) > 1 else '/root/repo/profiles/r2_precision_attribution.json'
+    out_path = sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, 'profiles', 'r2_precision_attribution.json')
     t0 = time.time()
     ref = run()
     flops = dict(FLOPS)

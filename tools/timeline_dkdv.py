@@ -1,10 +1,11 @@
 """Debug: per-phase clock64 timeline of one dK/dV CTA (library built with -DCTRLORA_TIMELINE)."""
 import ctypes
+import os
 import sys
 
 import torch
 
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ctrlora_b200 import _lib, ops  # noqa: E402
 from tools.profile_kernels import rnd  # noqa: E402
 
